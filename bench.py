@@ -4,6 +4,7 @@ sharded over N GPUs of one node (STRONG scaling: the global batch is fixed at 64
   python bench.py --gpus N --steps K --warmup W            # our arm (libmmg.so through the drop-in classes + parallel.generate_sharded)
   python bench.py --impl reference --gpus N --steps K ...  # the UNMODIFIED reference's MaskGit.generate() on the host cores (baseline/_ref)
   python bench.py --config C2|C4|C5                        # secondary configs of BASELINE.json (one JSON line each; C3 is the default)
+  python bench.py ... --dump-outputs DIR                   # C3: also write the last timed step's images to DIR/images.npy
 
 One "step" = one full generate() call over the rank's shard (18 decode steps + VAE decode + (N>1) one NCCL all-gather of
 the decoded images).  `value` is timed with the text embeddings already resident in HBM; `e2e` times the same public call
@@ -36,6 +37,7 @@ GFLOP_C4_IMAGE = 4026.0
 GFLOP_C5_IMAGE = 1178.9
 METRIC = "images/sec MaskGit.generate() 256x256 18-step CFG=3"
 REF_BATCH = 4                       # BASELINE.md section 4: the CPU arm runs B_cpu = 4 (CPU throughput is flat in B)
+DUMP_BYTES = 64 << 20               # --dump-outputs writes at most this much (the 64 images of C3 are 50 MB in fp32)
 
 
 def peaks():
@@ -161,7 +163,11 @@ def run_ours(args):
     sampler = ClockSampler(local) if rank == 0 else None
     if sampler:
         sampler.start()
-    ms, launches = timed_loop(dist, world, device, lambda: step(False), args.steps)
+    last = {}
+
+    def timed_step():
+        last["images"] = step(False)
+    ms, launches = timed_loop(dist, world, device, timed_step, args.steps)
     clocks = sampler.stop() if sampler else None
     step(True)
     ms_e2e, _ = timed_loop(dist, world, device, lambda: step(True), args.steps)
@@ -199,11 +205,26 @@ def run_ours(args):
             line["parity"] = teacher_forced_flip_rate(mg)
             line["gpu_eager_baseline"] = gpu_eager_baseline(device)
             line["cpu_baseline"] = cpu_baseline()
+        if args.dump_outputs:
+            dump_images(args.dump_outputs, last["images"])
     if world > 1:
         dist.barrier()
         dist.destroy_process_group()
     if rank == 0:
         print(json.dumps(line))
+
+
+def dump_images(directory, images):
+    """--dump-outputs: the images the timed generate() returned in its last timed step, as float32 DIR/images.npy, so that two builds run with
+    the same arguments (hence the same seeded weights, text embeddings and sampler seed) can be compared output for output.  A batch larger
+    than DUMP_BYTES (--global-batch) is cut to a fixed, seeded sample of whole images."""
+    import numpy as np
+    a = images.detach().float().cpu().numpy()
+    if a.nbytes > DUMP_BYTES:
+        keep = np.sort(np.random.default_rng(0).choice(a.shape[0], DUMP_BYTES // a[0].nbytes, replace=False))
+        a = a[keep]
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "images.npy"), a)
 
 
 def _gemm_flops(name, a):
@@ -626,7 +647,12 @@ if __name__ == "__main__":
     ap.add_argument("--no-extras", "--no-cpu-baseline", dest="no_extras", action="store_true",
                     help="skip cpu_baseline / parity / gpu_eager_baseline / hbm_kernels (N=1 extras)")
     ap.add_argument("--global-batch", type=int, default=GLOBAL_BATCH, help="experiments only; the benchmark config is 64")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="C3: write the images of the last timed step to DIR/images.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.config != "C3"):
+        ap.error("--dump-outputs applies to the C3 benchmark of this implementation")
     GLOBAL_BATCH = args.global_batch
     if args.impl == "reference":
         run_reference(args)

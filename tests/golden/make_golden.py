@@ -73,6 +73,13 @@ assert known["sched_256_18"] == [256, 254, 251, 246, 238, 229, 217, 204, 189, 17
 with open(os.path.join(HERE, "known_answers.json"), "w") as f:
     json.dump(known, f, indent=1)
 
+# ------------------------------------------------------------------ SHA-256 of the reference's modules (tests/test_abi.py checks baseline/_ref against them)
+import hashlib                                                      # noqa: E402
+pkg_dir = os.path.dirname(os.path.abspath(ref_t5.__file__))
+with open(os.path.join(HERE, "reference_sources.json"), "w") as f:
+    json.dump({n: hashlib.sha256(open(os.path.join(pkg_dir, n), "rb").read()).hexdigest() for n in sorted(os.listdir(pkg_dir)) if n.endswith(".py")},
+              f, indent=1)
+
 # ------------------------------------------------------------------ G1: config C1 — VAE dim=64 cb=512 on 4x3x32x32
 vae = VQGanVAE(dim=64, codebook_size=512).eval()
 fill(vae, shapes.vae_shapes(64, codebook_size=512), seed=11)

@@ -69,17 +69,17 @@ def test_decode_step_workspace_query_is_host_only():
 
 
 def test_baseline_ref_is_the_unmodified_reference():
-    """baseline/_ref (the reference arm of bench.py) is byte-identical to /root/reference wherever both exist (build container)."""
-    import filecmp
+    """baseline/_ref (the reference arm of bench.py) holds the unmodified reference: its modules are exactly those of the upstream package,
+    byte for byte, by the SHA-256 digests recorded from the upstream sources in tests/golden/reference_sources.json (make_golden.py)."""
+    import hashlib
+    import json
     import pytest
-    ref = "/root/reference/muse_maskgit_pytorch"
     inst = os.path.join(ROOT, "baseline", "_ref", "muse_maskgit_pytorch")
-    if not (os.path.isdir(ref) and os.path.isdir(inst)):
-        pytest.skip("needs /root/reference and baseline/_ref")
-    names = sorted(f for f in os.listdir(ref) if f.endswith(".py"))
-    assert names and names == sorted(f for f in os.listdir(inst) if f.endswith(".py"))
-    match, mismatch, errors = filecmp.cmpfiles(ref, inst, names, shallow=False)
-    assert not mismatch and not errors, (mismatch, errors)
+    if not os.path.isdir(inst):
+        pytest.skip("baseline/_ref is not installed (build() installs it only where the reference sources are available)")
+    want = json.load(open(os.path.join(ROOT, "tests", "golden", "reference_sources.json")))
+    got = {f: hashlib.sha256(open(os.path.join(inst, f), "rb").read()).hexdigest() for f in os.listdir(inst) if f.endswith(".py")}
+    assert want and got == want, sorted(f for f in set(got) | set(want) if got.get(f) != want.get(f))
 
 
 def test_pack_cache_digest_tracks_weights():
