@@ -188,7 +188,12 @@ int mmg_embed(const mmg_embed_args* a, void* stream);
  * Attention core: out[b, t, h*64:(h+1)*64] = softmax(scale * q.k^T + key_mask) v   with dh = 64.
  * q [BH, Tq, 64], k/v [BH, Tk_alloc, 64] already l2-normalised/scaled (epilogue MMG_EPI_QKV); key 0 is the null key.
  * replaces: Attend.forward / flash_attn (attend.py:66-140) + the head split/merge in Attention.forward
- * (muse_maskgit_pytorch.py:143-161).  key_mask: [B, Tk] uint8 (1 = attend) or NULL; masked logits = -FLT_MAX.     */
+ * (muse_maskgit_pytorch.py:143-161).  key_mask: [B, Tk - 1] uint8, one byte per real key 1 .. Tk-1 (1 = attend; the null key is never
+ * masked) or NULL; masked logits = -FLT_MAX.
+ * Padding: rows [Tk, Tk_alloc) of each k / v head may be read (the tensor-core kernels load whole key blocks, so the last block reads into
+ * the padding, or into the next head's rows) but never reach the output: they, like masked keys, get a weight of exactly 0.  They and the
+ * masked keys' rows must hold finite values: 0 * inf is NaN, and the kernels do not guard against it.  Zero padding (what MMG_EPI_QKV
+ * leaves) is fine.                                                                                                  */
 typedef struct {
   const void* q; const void* k; const void* v; void* out;
   const uint8_t* key_mask;

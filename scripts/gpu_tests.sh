@@ -22,4 +22,5 @@ runall models 900 tests/test_gpu_models.py
 runall aten_rng 600 tests/test_gpu_aten_rng.py
 runall full_config 900 tests/test_gpu_full_config.py
 runall fused_tail 600 tests/test_gpu_fused_tail.py
+runall attention_edges 600 tests/test_gpu_attention_edges.py
 cat $OUT/summary.txt
